@@ -2,7 +2,7 @@
 """bench.py -- the depth -> sort -> rasterise hot path on N B200s (BASELINE.json metric: frames/s and sorted
 Msplats/s at 1920x1080; HBM GB/s against the measured roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload bonsai|garden|synth16m]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload bonsai|garden|synth16m] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one viewer frame: full depth sort of every splat + projection + tile binning + front-to-back blend into an
@@ -42,6 +42,7 @@ WORKLOADS = {
 }
 SH_BYTES = {0: 0, 1: 18, 2: 48}
 ORBIT_DEGREES_PER_FRAME = 3.0
+DUMP_BUDGET_BYTES = 60_000_000        # --dump-outputs: data bytes of all arrays together (under 64 MB with the .npy headers)
 
 
 def workload_label(name: str) -> str:
@@ -142,6 +143,23 @@ def prepared_frames(v, workload: str, frame_format: int):
     return out
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: arrays = {name: (array, float dtype)} -> out_dir/<name>.npy.  The dtypes hold every value exactly (RGBA8 channels,
+    u32 indexes).  When the arrays together exceed DUMP_BUDGET_BYTES, each keeps the same share of its elements, a seeded sample of
+    flat positions: the same positions in every run of the same workload, so two builds' dumps compare element for element."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    total = sum(a.size * np.dtype(dt).itemsize for a, dt in arrays.values())
+    keep = min(1.0, DUMP_BUDGET_BYTES / total)
+    for name, (a, dt) in arrays.items():
+        out = a.astype(dt)
+        if keep < 1.0:
+            pos = np.sort(np.random.default_rng(0).choice(a.size, int(a.size * keep), replace=False))
+            out = out.reshape(-1)[pos]
+        np.save(d / f"{name}.npy", out)
+        print(f"[bench] {d / name}.npy: {out.size} of {a.size} elements of {name} {a.shape}, {np.dtype(dt).name}", file=sys.stderr)
+
+
 # ------------------------------------------------------------------------------------------------------------------------------
 def cpu_frame_seconds(workload: str, repeats: int):
     """The reference's CPU path: its own sorter (oracle/_ref, single-threaded like its one Web Worker; the C restatement when the
@@ -151,7 +169,6 @@ def cpu_frame_seconds(workload: str, repeats: int):
     from gaussiansplats3d_b200 import three_math as TM
     from gaussiansplats3d_b200.engine import Uniforms
     from gaussiansplats3d_b200.scenes import CAMERAS, pack_scene, synthetic_scene
-    oracle.build()
     threads = oracle.set_threads(os.cpu_count() or 1)
     n, sh, kind, seed, cam, w, h, orbit = WORKLOADS[workload]
     raw = synthetic_scene(n, seed=seed, kind=kind, sh_degree=sh)
@@ -322,6 +339,16 @@ def run_ours(args):
     barrier()
     launches = e.timings()["kernel_launches"] * K
     step_ms = np.array([ev0[i].elapsed_ms(ev1[i]) for i in range(K)])
+    if args.dump_outputs and rank == 0:     # the last timed step's picture (and, on one GPU, its draw order), read back untimed
+        if world > 1 and not peer:
+            gather.sync_to_torch()
+            picture = gather.image().cpu().numpy()
+        else:
+            picture = e.read_buffer(N.GS_BUF_FRAME, np.uint8, height * width * 4).reshape(height, width, 4)
+        arrays = {"frame_rgba8": (picture, np.float32)}
+        if world == 1:
+            arrays["sorted_indexes"] = (e.read_buffer(N.GS_BUF_SORTED_INDEXES, np.uint32, n), np.float32 if n <= 1 << 24 else np.float64)
+        dump_outputs(args.dump_outputs, arrays)
     total_ms = float(step_ms.sum())
     if dist is not None:
         t = torch.tensor([total_ms], device="cuda", dtype=torch.float64)
@@ -561,7 +588,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="bonsai", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (RGBA8 frame; one GPU: also the sorted indexes) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
     if args.impl == "reference":
         if args.steps is None:     # the CPU arm's frames take ~0.5 s each
             args.steps = 10

@@ -122,6 +122,13 @@ def sort_matrix(n=20000, seeds=(0,)):
     return out
 
 
+def property_case(seed, n, integer, mode, kind, frac, rbits, ties):
+    """(case, distance_map_range) of one property example: mode is "static", "dynamic" or "precomputed", the range is 2^rbits."""
+    c = sort_case(seed=seed, n=n, integer=integer, dynamic=(mode == "dynamic"), precomputed=(mode == "precomputed"), index_kind=kind,
+                  sort_frac=frac, ties=ties and mode != "precomputed")
+    return c, 1 << rbits
+
+
 RANGES = (1 << 10, 1 << 16, 1 << 20)
 
 
