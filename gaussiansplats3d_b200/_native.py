@@ -27,14 +27,15 @@ GS_OK, GS_ERR_BAD_ARG, GS_ERR_NO_DEVICE, GS_ERR_CUDA, GS_ERR_DEGENERATE, GS_ERR_
 GS_COV_F32, GS_COV_F16 = 0, 1
 GS_SH_NONE, GS_SH_F16, GS_SH_U8, GS_SH_F32 = 0, 1, 2, 3
 GS_FRAME_RGBA32F, GS_FRAME_RGBA8 = 0, 1
-GS_BUF_SORTED_INDEXES, GS_BUF_FRAME, GS_BUF_CENTERS, GS_BUF_DISTANCES, GS_BUF_SPLAT_RECORDS, GS_BUF_INDEXES_TO_SORT, GS_BUF_CENTERS_COLORS, GS_BUF_COVARIANCES, GS_BUF_SH = range(9)
+GS_BUF_SORTED_INDEXES, GS_BUF_FRAME, GS_BUF_CENTERS, GS_BUF_DISTANCES, GS_BUF_SPLAT_RECORDS, GS_BUF_INDEXES_TO_SORT, GS_BUF_CENTERS_COLORS, GS_BUF_COVARIANCES, GS_BUF_SH, GS_BUF_SCALE_ROTATIONS = range(10)
+GS_RENDER_MODE_3D, GS_RENDER_MODE_2D = 0, 1
 
 
 class gs_config(C.Structure):
     _fields_ = [
         ("struct_size", C.c_uint32), ("device", C.c_int32), ("max_splat_count", C.c_uint32),
         ("distance_map_range", C.c_uint32), ("integer_based_sort", C.c_uint8), ("dynamic_mode", C.c_uint8),
-        ("reserved0", C.c_uint8 * 2), ("max_width", C.c_uint32), ("max_height", C.c_uint32),
+        ("splat_render_mode", C.c_uint8), ("reserved0", C.c_uint8), ("max_width", C.c_uint32), ("max_height", C.c_uint32),
         ("rank", C.c_uint32), ("world_size", C.c_uint32),
     ]
 
@@ -52,7 +53,7 @@ class gs_splat_data(C.Structure):
     _fields_ = [
         ("struct_size", C.c_uint32), ("from_", C.c_uint32), ("count", C.c_uint32), ("centers_colors", C.c_void_p),
         ("covariances", C.c_void_p), ("cov_format", C.c_int32), ("spherical_harmonics", C.c_void_p),
-        ("sh_format", C.c_int32), ("sh_degree", C.c_uint32), ("scene_indexes", C.c_void_p),
+        ("sh_format", C.c_int32), ("sh_degree", C.c_uint32), ("scene_indexes", C.c_void_p), ("scale_rotations", C.c_void_p),
     ]
 
 
@@ -90,6 +91,15 @@ class gs_projected_splat(C.Structure):
 PROJECTED_DTYPE = np.dtype([(n, np.float32) for n in ("cx", "cy", "b1x", "b1y", "b2x", "b2y", "r", "g", "b", "a", "ndc_z")] + [("valid", np.uint32)])
 
 
+class gs_projected_surfel(C.Structure):
+    _fields_ = [("T", C.c_float * 9)] + [(n, C.c_float) for n in ("qcx", "qcy", "cx", "cy", "h1x", "h1y", "h2x", "h2y", "r", "g", "b", "a", "ndc_z")] + \
+        [("branch", C.c_uint32), ("valid", C.c_uint32)]
+
+
+PROJECTED_SURFEL_DTYPE = np.dtype([("T", np.float32, (9,))] + [(n, np.float32) for n in ("qcx", "qcy", "cx", "cy", "h1x", "h1y", "h2x", "h2y", "r", "g", "b", "a", "ndc_z")]
+                                  + [("branch", np.uint32), ("valid", np.uint32)])
+
+
 class gs_timings(C.Structure):
     _fields_ = [
         ("depth_ms", C.c_float), ("bucket_ms", C.c_float), ("scatter_ms", C.c_float), ("sort_total_ms", C.c_float),
@@ -120,7 +130,7 @@ EXPORTED_SYMBOLS = [
     "gs_abi_version", "gs_status_string", "gs_last_error_message", "gs_device_count", "gs_sort_indexes", "sortIndexes", "gs_dropin_release",
     "gs_create", "gs_destroy", "gs_upload_centers", "gs_sort", "gs_compute_distances", "gs_upload_splat_data",
     "gs_render", "gs_frame", "gs_buffer_dev", "gs_stream", "gs_synchronize", "gs_host_alloc", "gs_host_free",
-    "gs_read_projected", "gs_last_timings", "gs_frame_async", "gs_frame_begin", "gs_frame_end", "gs_upload_splat_tree", "gs_gather_for_sort", "gs_flush_l2", "gs_event_create", "gs_event_record",
+    "gs_read_projected", "gs_read_projected_2d", "gs_last_timings", "gs_frame_async", "gs_frame_begin", "gs_frame_end", "gs_upload_splat_tree", "gs_gather_for_sort", "gs_flush_l2", "gs_event_create", "gs_event_record",
     "gs_event_elapsed_ms", "gs_event_destroy", "gs_set_profiling", "gs_kernel_timings", "gs_set_graph_enabled", "gs_upload_ksplat", "gs_read_buffer", "gs_peer_export", "gs_peer_attach",
     "gs_shard_export", "gs_shard_attach", "gs_shard_attach_local", "gs_sort_sharded", "gs_sort_sharded_async", "gs_sort_sharded_finish",
 ]
@@ -179,6 +189,8 @@ def load() -> C.CDLL:
     lib.gs_host_free.argtypes = [vp]
     lib.gs_read_projected.restype = C.c_int
     lib.gs_read_projected.argtypes = [vp, vp, u32]
+    lib.gs_read_projected_2d.restype = C.c_int
+    lib.gs_read_projected_2d.argtypes = [vp, vp, u32]
     lib.gs_last_timings.restype = C.c_int
     lib.gs_last_timings.argtypes = [vp, C.POINTER(gs_timings)]
     lib.gs_upload_splat_tree.restype = C.c_int

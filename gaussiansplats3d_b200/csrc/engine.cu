@@ -213,6 +213,7 @@ extern "C" int gs_create(const gs_config *cfg, gs_engine **out) {
     if (c.distance_map_range < 2 || c.distance_map_range > (1u << 24)) return fail(GS_ERR_BAD_ARG, "distance_map_range %u outside [2, 2^24]", c.distance_map_range);
     if (c.world_size == 0) { c.world_size = 1; c.rank = 0; }
     if (c.rank >= c.world_size) return fail(GS_ERR_BAD_ARG, "rank %u >= world_size %u", c.rank, c.world_size);
+    if (c.splat_render_mode > GS_RENDER_MODE_2D) return fail(GS_ERR_BAD_ARG, "splat_render_mode %u is neither ThreeD (0) nor TwoD (1)", (unsigned)c.splat_render_mode);
     int ndev = gs_device_count();
     if (ndev <= 0) return fail(GS_ERR_NO_DEVICE, "no CUDA device visible: libgsplat_b200 has no CPU path");
     if (c.device < 0 || c.device >= ndev) return fail(GS_ERR_BAD_ARG, "device %d not in [0,%d)", c.device, ndev);
@@ -874,7 +875,11 @@ extern "C" int gs_upload_splat_data(gs_engine *e, const gs_splat_data *d) {
     int rc = check_engine(e);
     if (rc) return rc;
     if (!d) return fail(GS_ERR_BAD_ARG, "gs_upload_splat_data: null");
-    rc = raster_upload(e->rs, e->cfg, *d, e->stream);
+    // callers built against the shorter struct (no scale_rotations) are recognised by struct_size; 0 means that older layout
+    gs_splat_data dd{};
+    const size_t old_size = offsetof(gs_splat_data, scale_rotations);
+    memcpy(&dd, d, std::min<size_t>(d->struct_size ? d->struct_size : old_size, sizeof(gs_splat_data)));
+    rc = raster_upload(e->rs, e->cfg, dd, e->stream);
     if (rc) return rc;
     CU(cudaStreamSynchronize(e->stream));
     return GS_OK;
@@ -997,7 +1002,7 @@ static int enqueue_frame(gs_engine *e, const gs_sort_params *s, const gs_uniform
     if (use_graph) {
         const unsigned long long key[8] = {q.render_count, q.sort_count, ((unsigned long long)rp.width << 32) | rp.height,
                                            ((unsigned long long)rp.frame_format << 8) | (unsigned long long)(rp.flip_y ? 1 : 0) | ((unsigned long long)q.use_precomputed_distances << 4),
-                                           (unsigned long long)(uintptr_t)d_idx, ((unsigned long long)e->rs.cov_format << 16) | ((unsigned long long)e->rs.sh_format << 8) | e->rs.sh_degree,
+                                           (unsigned long long)(uintptr_t)d_idx, ((unsigned long long)e->rs.render_mode << 32) | ((unsigned long long)e->rs.cov_format << 16) | ((unsigned long long)e->rs.sh_format << 8) | e->rs.sh_degree,
                                            e->rs.uploaded, ((unsigned long long)rp.render_count << 1) | (subset ? 1ull : 0ull)};
         if ((rc = upload_frame_params(e, q.model_view_proj, *u, rp))) return rc;
         cudaGraphExec_t &gexec = e->rs.frame_parity ? e->graph_exec_alt : e->graph_exec;      // one instantiated graph per target frame buffer
@@ -1324,12 +1329,13 @@ extern "C" int gs_upload_ksplat(gs_engine *e, const void *data, size_t bytes, co
     // storage formats of the "textures" (SplatMesh.js:1064-1066: SH kept at compression level max(1, file level))
     RasterState &rs = e->rs;
     rs.uploaded = 0;
-    rs.cov_format = o.half_covariances ? GS_COV_F16 : GS_COV_F32;
+    const bool two_d = rs.render_mode == GS_RENDER_MODE_2D;   // scale/rotation texture instead of covariances (half_covariances unused)
+    rs.cov_format = (o.half_covariances && !two_d) ? GS_COV_F16 : GS_COV_F32;
     rs.sh_degree = min_degree;
     rs.sh_format = min_degree ? (level == 2 ? GS_SH_U8 : GS_SH_F16) : GS_SH_NONE;
     const size_t n = e->cfg.max_splat_count, ncomp_out = min_degree == 2 ? 24 : (min_degree == 1 ? 9 : 0);
     cudaError_t ce;
-    if ((ce = rs.cov.ensure(n * (o.half_covariances ? 12 : 24) + 16)) != cudaSuccess) return fail(GS_ERR_CUDA, "cudaMalloc -> %s", cudaGetErrorString(ce));
+    if (!two_d && (ce = rs.cov.ensure(n * (o.half_covariances ? 12 : 24) + 16)) != cudaSuccess) return fail(GS_ERR_CUDA, "cudaMalloc -> %s", cudaGetErrorString(ce));
     if (ncomp_out && (ce = rs.sh.ensure(n * ncomp_out * (level == 2 ? 1 : 2) + 16)) != cudaSuccess) return fail(GS_ERR_CUDA, "cudaMalloc -> %s", cudaGetErrorString(ce));
     DevBuf<unsigned char> d_file; DevBuf<uint32_t> d_pre; DevBuf<KTransform> d_xf;
     struct Scratch {   // the staged file and the bucket prefixes live for this call only, whichever way it returns
@@ -1356,8 +1362,14 @@ extern "C" int gs_upload_ksplat(gs_engine *e, const void *data, size_t bytes, co
         P.sh_degree_out = (int)min_degree;
         P.minimum_alpha = o.minimum_alpha; P.half_cov = o.half_covariances; P.integer_centers = e->cfg.integer_based_sort; P.write_sort_centers = o.upload_sort_centers;
         if (P.count) {
-            if (o.has_transform) k_ksplat_decode<true><<<(P.count + 127) / 128, 128, 0, st>>>(d_file.p, P, d_pre.p + at, rs.cc.p, rs.cov.p, rs.sh.p, e->centers.p, d_xf.p);
-            else k_ksplat_decode<false><<<(P.count + 127) / 128, 128, 0, st>>>(d_file.p, P, d_pre.p + at, rs.cc.p, rs.cov.p, rs.sh.p, e->centers.p, nullptr);
+            const dim3 grid((P.count + 127) / 128);
+            if (two_d) {
+                if (o.has_transform) k_ksplat_decode<true, true><<<grid, 128, 0, st>>>(d_file.p, P, d_pre.p + at, rs.cc.p, nullptr, rs.sh.p, e->centers.p, d_xf.p, rs.srot.p);
+                else k_ksplat_decode<false, true><<<grid, 128, 0, st>>>(d_file.p, P, d_pre.p + at, rs.cc.p, nullptr, rs.sh.p, e->centers.p, nullptr, rs.srot.p);
+            } else {
+                if (o.has_transform) k_ksplat_decode<true, false><<<grid, 128, 0, st>>>(d_file.p, P, d_pre.p + at, rs.cc.p, rs.cov.p, rs.sh.p, e->centers.p, d_xf.p, nullptr);
+                else k_ksplat_decode<false, false><<<grid, 128, 0, st>>>(d_file.p, P, d_pre.p + at, rs.cc.p, rs.cov.p, rs.sh.p, e->centers.p, nullptr, nullptr);
+            }
         }
         at += prefixes[i].size();
     }
@@ -1387,6 +1399,7 @@ extern "C" int gs_read_buffer(gs_engine *e, int id, void *out, size_t offset, si
         case GS_BUF_CENTERS_COLORS: p = (const unsigned char *)e->rs.cc.p; cap = e->rs.cc.n * 16; break;
         case GS_BUF_COVARIANCES: p = e->rs.cov.p; cap = e->rs.cov.n; break;
         case GS_BUF_SH: p = e->rs.sh.p; cap = e->rs.sh.n; break;
+        case GS_BUF_SCALE_ROTATIONS: p = (const unsigned char *)e->rs.srot.p; cap = e->rs.srot.n * 4; break;
         default: { void *q = nullptr; if ((rc = gs_buffer_dev(e, id, &q, &cap))) return rc; p = (const unsigned char *)q; }
     }
     if (!p || offset + bytes > cap) return fail(GS_ERR_CAPACITY, "gs_read_buffer: [%zu,%zu) outside the %zu-byte buffer", offset, offset + bytes, cap);
@@ -1405,6 +1418,17 @@ extern "C" int gs_read_projected(gs_engine *e, gs_projected_splat *out, uint32_t
     return GS_OK;
 }
 
+extern "C" int gs_read_projected_2d(gs_engine *e, gs_projected_surfel *out, uint32_t count) {
+    int rc = check_engine(e);
+    if (rc) return rc;
+    if (!out) return fail(GS_ERR_BAD_ARG, "gs_read_projected_2d: null");
+    if (e->pipe_inflight()) return fail(GS_ERR_NOT_READY, "gs_read_projected_2d: pipelined frames are in flight (gs_frame_end first)");
+    rc = raster_read_projected_2d(e->rs, out, count, e->stream);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(e->stream));
+    return GS_OK;
+}
+
 extern "C" int gs_buffer_dev(gs_engine *e, int id, void **ptr, size_t *bytes) {
     if (!e || !ptr) return fail(GS_ERR_BAD_ARG, "gs_buffer_dev: null");
     size_t b = 0;
@@ -1413,7 +1437,10 @@ extern "C" int gs_buffer_dev(gs_engine *e, int id, void **ptr, size_t *bytes) {
         case GS_BUF_FRAME: *ptr = raster_frame_ptr(e->rs, e->rs.last_format); b = e->rs.last_frame_bytes; break;
         case GS_BUF_CENTERS: *ptr = e->centers.p; b = e->centers.n * 16; break;
         case GS_BUF_DISTANCES: *ptr = e->dist.p; b = e->dist.n * 4; break;
-        case GS_BUF_SPLAT_RECORDS: *ptr = e->rs.records.p; b = e->rs.records.n * sizeof(SplatRecord); break;
+        case GS_BUF_SPLAT_RECORDS:
+            if (e->rs.render_mode == GS_RENDER_MODE_2D) { *ptr = e->rs.surfels.p; b = e->rs.surfels.n * sizeof(SurfelRecord); }
+            else { *ptr = e->rs.records.p; b = e->rs.records.n * sizeof(SplatRecord); }
+            break;
         case GS_BUF_INDEXES_TO_SORT: *ptr = e->indexes.p; b = e->indexes.n * 4; break;
         default: return fail(GS_ERR_BAD_ARG, "unknown buffer id %d", id);
     }

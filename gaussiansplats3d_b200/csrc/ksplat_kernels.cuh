@@ -50,12 +50,79 @@ __device__ __forceinline__ uint16_t to_half_three(float val) {
     return (uint16_t)((base | sign) + (mant >> shift));
 }
 
+// TwoD render mode: SplatBuffer.fillSplatScaleRotationArray (SplatBuffer.js:349-438) for one splat, in float64 with three.js's operation
+// order (unfused): quaternion.normalize(); with a scene transform, transform * R * S (Matrix4.multiplyMatrices: the R*S and S*I products
+// are exact, the zero fourth-row terms add exact zeros) -> Matrix4.decompose -> normalize; ensurePositiveW.  sz is the SplatMesh
+// override (1 read at the file's compression level, SplatMesh.js:1856-1863).  Out: f32 [sx sy sz qx qy qz].
+__device__ __forceinline__ void ksplat_scale_rotation(const double *T, double sx, double sy, double sz, double x, double y, double z, double w,
+                                                      float *out) {
+    auto normalize = [](double &x, double &y, double &z, double &w) {
+        const double ln = __dsqrt_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z)), __dmul_rn(w, w)));
+        if (ln == 0.0) { x = y = z = 0.0; w = 1.0; return; }
+        const double il = __ddiv_rn(1.0, ln);
+        x = __dmul_rn(x, il); y = __dmul_rn(y, il); z = __dmul_rn(z, il); w = __dmul_rn(w, il);
+    };
+    normalize(x, y, z, w);
+    if (T) {
+        const double x2 = __dadd_rn(x, x), y2 = __dadd_rn(y, y), z2 = __dadd_rn(z, z);
+        const double xx = __dmul_rn(x, x2), xy = __dmul_rn(x, y2), xz = __dmul_rn(x, z2), yy = __dmul_rn(y, y2), yz = __dmul_rn(y, z2), zz = __dmul_rn(z, z2);
+        const double wx = __dmul_rn(w, x2), wy = __dmul_rn(w, y2), wz = __dmul_rn(w, z2);
+        const double R[3][3] = {{__dsub_rn(1.0, __dadd_rn(yy, zz)), __dsub_rn(xy, wz), __dadd_rn(xz, wy)},
+                                {__dadd_rn(xy, wz), __dsub_rn(1.0, __dadd_rn(xx, zz)), __dsub_rn(yz, wx)},
+                                {__dsub_rn(xz, wy), __dadd_rn(yz, wx), __dsub_rn(1.0, __dadd_rn(xx, yy))}};
+        const double sc[3] = {sx, sy, sz};
+        double RS[3][3], m[3][3];
+#pragma unroll
+        for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int j = 0; j < 3; ++j) RS[i][j] = __dmul_rn(R[i][j], sc[j]);
+#pragma unroll
+        for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int j = 0; j < 3; ++j)
+                m[i][j] = __dadd_rn(__dadd_rn(__dmul_rn(T[i], RS[0][j]), __dmul_rn(T[4 + i], RS[1][j])), __dmul_rn(T[8 + i], RS[2][j]));
+        double dsx = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(m[0][0], m[0][0]), __dmul_rn(m[1][0], m[1][0])), __dmul_rn(m[2][0], m[2][0])));
+        const double dsy = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(m[0][1], m[0][1]), __dmul_rn(m[1][1], m[1][1])), __dmul_rn(m[2][1], m[2][1])));
+        const double dsz = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(m[0][2], m[0][2]), __dmul_rn(m[1][2], m[1][2])), __dmul_rn(m[2][2], m[2][2])));
+        // Matrix4.determinant: only its sign is used (the affine fourth row leaves the n44 term)
+        const double det = m[0][0] * (m[1][1] * m[2][2] - m[1][2] * m[2][1]) - m[0][1] * (m[1][0] * m[2][2] - m[1][2] * m[2][0]) +
+                           m[0][2] * (m[1][0] * m[2][1] - m[1][1] * m[2][0]);
+        if (det < 0) dsx = -dsx;
+        const double is[3] = {__ddiv_rn(1.0, dsx), __ddiv_rn(1.0, dsy), __ddiv_rn(1.0, dsz)};
+        double r[3][3];
+#pragma unroll
+        for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int j = 0; j < 3; ++j) r[i][j] = __dmul_rn(m[i][j], is[j]);
+        const double t = __dadd_rn(__dadd_rn(r[0][0], r[1][1]), r[2][2]);   // Quaternion.setFromRotationMatrix
+        if (t > 0) {
+            const double k = __ddiv_rn(0.5, __dsqrt_rn(__dadd_rn(t, 1.0)));
+            w = __ddiv_rn(0.25, k); x = __dmul_rn(__dsub_rn(r[2][1], r[1][2]), k); y = __dmul_rn(__dsub_rn(r[0][2], r[2][0]), k); z = __dmul_rn(__dsub_rn(r[1][0], r[0][1]), k);
+        } else if (r[0][0] > r[1][1] && r[0][0] > r[2][2]) {
+            const double k = __dmul_rn(2.0, __dsqrt_rn(__dsub_rn(__dsub_rn(__dadd_rn(1.0, r[0][0]), r[1][1]), r[2][2])));
+            w = __ddiv_rn(__dsub_rn(r[2][1], r[1][2]), k); x = __dmul_rn(0.25, k); y = __ddiv_rn(__dadd_rn(r[0][1], r[1][0]), k); z = __ddiv_rn(__dadd_rn(r[0][2], r[2][0]), k);
+        } else if (r[1][1] > r[2][2]) {
+            const double k = __dmul_rn(2.0, __dsqrt_rn(__dsub_rn(__dsub_rn(__dadd_rn(1.0, r[1][1]), r[0][0]), r[2][2])));
+            w = __ddiv_rn(__dsub_rn(r[0][2], r[2][0]), k); x = __ddiv_rn(__dadd_rn(r[0][1], r[1][0]), k); y = __dmul_rn(0.25, k); z = __ddiv_rn(__dadd_rn(r[1][2], r[2][1]), k);
+        } else {
+            const double k = __dmul_rn(2.0, __dsqrt_rn(__dsub_rn(__dsub_rn(__dadd_rn(1.0, r[2][2]), r[0][0]), r[1][1])));
+            w = __ddiv_rn(__dsub_rn(r[1][0], r[0][1]), k); x = __ddiv_rn(__dadd_rn(r[0][2], r[2][0]), k); y = __ddiv_rn(__dadd_rn(r[1][2], r[2][1]), k); z = __dmul_rn(0.25, k);
+        }
+        normalize(x, y, z, w);
+        sx = dsx; sy = dsy; sz = dsz;
+    }
+    const double flip = w < 0 ? -1.0 : 1.0;   // ensurePositiveW
+    out[0] = (float)sx; out[1] = (float)sy; out[2] = (float)sz;
+    out[3] = (float)(x * flip); out[4] = (float)(y * flip); out[5] = (float)(z * flip);
+}
+
 // XF: bake the scene transform (centre.applyMatrix4 :340-342, T3 (M M^T) T3^T :461-466, SH decode -> rotate -> re-encode :663-716).
-template <bool XF>
+// SR (TwoD engines): write the scale/rotation texture `srot` (6 x f32 per splat) instead of covariances.
+template <bool XF, bool SR>
 __global__ void __launch_bounds__(128)
 k_ksplat_decode(const unsigned char *__restrict__ file, KSectionParams P, const uint32_t *__restrict__ partial_prefix,
                 uint4 *__restrict__ cc, void *__restrict__ cov, void *__restrict__ sh_out, int4 *__restrict__ sort_centers,
-                const KTransform *__restrict__ xf) {
+                const KTransform *__restrict__ xf, float *__restrict__ srot) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= P.count) return;
     const unsigned char *rec = file + P.data_base + (size_t)i * P.bytes_per_splat;
@@ -111,8 +178,16 @@ k_ksplat_decode(const unsigned char *__restrict__ file, KSectionParams P, const 
                                         (int)floor(__dmul_rn((double)c[2], 1000.0) + 0.5), 1000);
         } else sort_centers[g] = make_int4(__float_as_int(c[0]), __float_as_int(c[1]), __float_as_int(c[2]), __float_as_int(1.0f));
     }
+    if (SR) {
+        // the z scale override 1 goes through toUncompressedFloat at the file's level: fromHalfFloat(1) = 2^-24 at levels 1 and 2
+        const double sz = P.level == 0 ? 1.0 : 5.9604644775390625e-08;
+        float o[6];
+        ksplat_scale_rotation(XF ? xf->t : nullptr, (double)s[0], (double)s[1], sz, (double)qx, (double)qy, (double)qz, (double)qw, o);
+        float2 *d = reinterpret_cast<float2 *>(srot + (size_t)g * 6);
+        d[0] = make_float2(o[0], o[1]); d[1] = make_float2(o[2], o[3]); d[2] = make_float2(o[4], o[5]);
+    }
     // ---- covariance = (R S)(R S)^T in float64, three.js operation order ---------------------------------------------------
-    {
+    if (!SR) {
         const double x = qx, y = qy, z = qz, w = qw;
         const double x2 = __dadd_rn(x, x), y2 = __dadd_rn(y, y), z2 = __dadd_rn(z, z);
         const double xx = __dmul_rn(x, x2), xy = __dmul_rn(x, y2), xz = __dmul_rn(x, z2), yy = __dmul_rn(y, y2), yz = __dmul_rn(y, z2), zz = __dmul_rn(z, z2);

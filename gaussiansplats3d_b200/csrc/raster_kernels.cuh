@@ -1380,6 +1380,10 @@ __global__ void k_export_projected(const SplatRecord *__restrict__ rec, const us
     out[s] = o;
 }
 
+} // namespace gs
+#include "surfel_kernels.cuh"   // the 2D (surfel) render mode's projection and blend
+namespace gs {
+
 // ---------------------------------------------------------------------------------------------------------------
 // Host side of the rasteriser
 template <typename T> struct RBuf {
@@ -1397,6 +1401,7 @@ template <typename T> struct RBuf {
 };
 
 struct RasterState {
+    int render_mode = GS_RENDER_MODE_3D;   // gs_config.splat_render_mode, fixed at create time
     RBuf<uint4> cc;
     RBuf<unsigned char> cov, sh;
     RBuf<uint32_t> scene_idx;
@@ -1404,6 +1409,9 @@ struct RasterState {
     uint32_t sh_degree = 0, uploaded = 0;
     bool have_scene_idx = false;
     RBuf<SplatRecord> records;
+    RBuf<float> srot;           // 2D: scale/rotation texture, 6 x f32 per splat
+    RBuf<SurfelRecord> surfels; // 2D: projected records (instead of `records`)
+    RBuf<gs_projected_surfel> exported2d;
     RBuf<ushort4> rects;
     RBuf<uint32_t> block_sums; // coarse instances per chunk of draw ranks
     RBuf<uint32_t> warp_sums;  // ... and per warp (256 draw ranks) inside the chunk
@@ -1460,15 +1468,18 @@ static inline char *raster_err() { return g_gs_err; }
 
 static int raster_init(RasterState &rs, const gs_config &c, int sm_count) {
     rs.sm_count = sm_count;
+    rs.render_mode = c.splat_render_mode;
     const size_t n = c.max_splat_count ? c.max_splat_count : 1;
     RCU(rs.rctl.ensure(1));
+    RCU(cudaMemset(rs.rctl.p, 0, sizeof(RasterControl)));   // k_raster_init resets the per-frame fields only (peer flags, frame count)
     RCU(rs.sctl.ensure(1));
     RCU(rs.dyn.ensure(2));          // per-frame parameter blocks: one per frame-buffer parity (pipelined frames upload them off-stream)
     RCU(rs.projp.ensure(2));
     RCU(cudaMemset(rs.dyn.p, 0, 2 * sizeof(DynamicUniforms)));
     if (c.max_width && c.max_height) {
         RCU(rs.cc.ensure(n));
-        RCU(rs.records.ensure(n));
+        if (rs.render_mode == GS_RENDER_MODE_2D) { RCU(rs.surfels.ensure(n)); RCU(rs.srot.ensure(6 * n)); }
+        else RCU(rs.records.ensure(n));
         RCU(rs.rects.ensure(n));
         RCU(rs.block_sums.ensure((n + kBinTile - 1) / kBinTile + 1));
         RCU(rs.warp_sums.ensure(((n + kBinTile - 1) / kBinTile + 1) * (kBinThreads / 32)));
@@ -1506,6 +1517,7 @@ static int raster_init(RasterState &rs, const gs_config &c, int sm_count) {
 
 static void raster_release(RasterState &rs) {
     rs.cc.release(); rs.cov.release(); rs.sh.release(); rs.scene_idx.release(); rs.records.release(); rs.rects.release();
+    rs.srot.release(); rs.surfels.release(); rs.exported2d.release();
     rs.block_sums.release(); rs.warp_sums.release(); rs.super_sums.release(); rs.ikeys[0].release(); rs.ikeys[1].release(); rs.ivals[0].release(); rs.ivals[1].release();
     rs.list.release(); rs.ranges.release(); rs.rctl.release(); rs.sctl.release(); rs.tile_hist.release(); rs.bin_hist.release(); rs.bin_totals.release(); rs.rect_by_rank.release(); rs.tile_order.release();
     rs.dyn.release(); rs.projp.release(); rs.frame.release(); rs.frame_alt.release(); rs.peer_sync_local.release(); rs.exported.release();
@@ -1514,7 +1526,10 @@ static void raster_release(RasterState &rs) {
 static int raster_upload(RasterState &rs, const gs_config &c, const gs_splat_data &d, cudaStream_t st) {
     if (!c.max_width || !c.max_height) { snprintf(raster_err(), 512, "engine created without a framebuffer (max_width/max_height = 0)"); return GS_ERR_NOT_READY; }
     if ((uint64_t)d.from + d.count > c.max_splat_count) { snprintf(raster_err(), 512, "splat data [%u,%u) exceeds max_splat_count %u", d.from, d.from + d.count, c.max_splat_count); return GS_ERR_CAPACITY; }
-    if (!d.centers_colors || !d.covariances) { snprintf(raster_err(), 512, "gs_upload_splat_data: null centers_colors/covariances"); return GS_ERR_BAD_ARG; }
+    const bool two_d = rs.render_mode == GS_RENDER_MODE_2D;
+    if (!d.centers_colors) { snprintf(raster_err(), 512, "gs_upload_splat_data: null centers_colors"); return GS_ERR_BAD_ARG; }
+    if (!two_d && !d.covariances) { snprintf(raster_err(), 512, "gs_upload_splat_data: null covariances"); return GS_ERR_BAD_ARG; }
+    if (two_d && !d.scale_rotations) { snprintf(raster_err(), 512, "gs_upload_splat_data: a TwoD (surfel) engine needs scale_rotations (6 floats per splat)"); return GS_ERR_BAD_ARG; }
     if (d.sh_degree > 2) { snprintf(raster_err(), 512, "sh_degree %u > 2", d.sh_degree); return GS_ERR_BAD_ARG; }
     const size_t n = c.max_splat_count;
     const size_t cov_elt = d.cov_format == GS_COV_F16 ? 12 : 24;
@@ -1527,13 +1542,14 @@ static int raster_upload(RasterState &rs, const gs_config &c, const gs_splat_dat
     rs.cov_format = d.cov_format;
     rs.sh_degree = d.sh_degree;
     rs.sh_format = ncomp ? d.sh_format : GS_SH_NONE;
-    RCU(rs.cov.ensure(n * cov_elt + 16));
+    if (!two_d) RCU(rs.cov.ensure(n * cov_elt + 16));
     if (ncomp) {
         if (!d.spherical_harmonics) { snprintf(raster_err(), 512, "sh_degree %u without spherical_harmonics", d.sh_degree); return GS_ERR_BAD_ARG; }
         RCU(rs.sh.ensure(n * sh_elt + 16));
     }
     RCU(cudaMemcpyAsync(rs.cc.p + d.from, d.centers_colors, (size_t)d.count * 16, cudaMemcpyHostToDevice, st));
-    RCU(cudaMemcpyAsync(rs.cov.p + (size_t)d.from * cov_elt, d.covariances, (size_t)d.count * cov_elt, cudaMemcpyHostToDevice, st));
+    if (two_d) RCU(cudaMemcpyAsync(rs.srot.p + (size_t)d.from * 6, d.scale_rotations, (size_t)d.count * 24, cudaMemcpyHostToDevice, st));
+    else RCU(cudaMemcpyAsync(rs.cov.p + (size_t)d.from * cov_elt, d.covariances, (size_t)d.count * cov_elt, cudaMemcpyHostToDevice, st));
     if (ncomp) RCU(cudaMemcpyAsync(rs.sh.p + (size_t)d.from * sh_elt, d.spherical_harmonics, (size_t)d.count * sh_elt, cudaMemcpyHostToDevice, st));
     if (d.scene_indexes) {
         RCU(rs.scene_idx.ensure(n));
@@ -1559,6 +1575,20 @@ static void launch_project(RasterState &rs, uint32_t count, cudaStream_t st) {
         default: GS_PROJ(GS_SH_NONE); break;
     }
 #undef GS_PROJ
+}
+
+template <bool EXPORT>
+static void launch_project2d(RasterState &rs, uint32_t count, cudaStream_t st, gs_projected_surfel *exp) {
+    const int blocks = (int)((count + kProjThreads - 1) / kProjThreads);
+    const uint32_t *sc = rs.have_scene_idx ? rs.scene_idx.p : nullptr;
+#define GS_PROJ2D(FMT) gs_launch(k_project2d<FMT, EXPORT>, blocks, kProjThreads, 0, st, rs.cc.p, rs.srot.p, rs.sh.p, (int)rs.sh_degree, sc, rs.dyn.p + rs.frame_parity, rs.projp.p + rs.frame_parity, count, rs.surfels.p, rs.rects.p, rs.rctl.p, exp)
+    switch (rs.sh_format) {
+        case GS_SH_F16: GS_PROJ2D(GS_SH_F16); break;
+        case GS_SH_U8: GS_PROJ2D(GS_SH_U8); break;
+        case GS_SH_F32: GS_PROJ2D(GS_SH_F32); break;
+        default: GS_PROJ2D(GS_SH_NONE); break;
+    }
+#undef GS_PROJ2D
 }
 
 // Fine-tile edge for a frame: 16 px while that gives at most 256 coarse tiles (8 x 4 fine tiles each: one counting-sort pass with 8-bit
@@ -1626,9 +1656,15 @@ static int raster_render(RasterState &rs, const gs_config &c, const gs_uniforms 
         // picture is earlier in stream order), so their blends never wait for rank 0's own sort + binning
         if (world > 1 && rs.peer_root) { k_peer_release<<<1, 1, 0, st>>>(rs.peer_sync, rs.rctl.p, (uint32_t)(rs.frame_parity && rs.frame_half2)); ++launches; }
         const uint32_t count = rs.uploaded;
-        if (rs.cov_format == GS_COV_F16) launch_project<true>(rs, count, st); else launch_project<false>(rs, count, st);
-        ++launches;
-        prof.mark("k_project", st);
+        if (rs.render_mode == GS_RENDER_MODE_2D) {
+            launch_project2d<false>(rs, count, st, nullptr);
+            ++launches;
+            prof.mark("k_project2d", st);
+        } else {
+            if (rs.cov_format == GS_COV_F16) launch_project<true>(rs, count, st); else launch_project<false>(rs, count, st);
+            ++launches;
+            prof.mark("k_project", st);
+        }
         if (record_events) RCU(cudaEventRecord(ev_project, st));
     }
     if (!(phases & 2)) { tm.kernel_launches = launches; return GS_OK; }
@@ -1682,7 +1718,19 @@ static int raster_render(RasterState &rs, const gs_config &c, const gs_uniforms 
             target = rs.peer_frame;
         }
         const uint32_t grid = ncoarse * kFinePerCoarse;
-        if (rs.blend_version >= 2 || tshift != kTileShift) {
+        if (rs.render_mode == GS_RENDER_MODE_2D) {
+            const bool to_peer = peer_mode && rs.peer_attached;
+            const StatusSnapshot snap{rs.snap_sort_ctl, reinterpret_cast<const uint32_t *>(rs.rctl.p),
+                                      (rs.snap_base && rs.snap_sort_ctl) ? rs.snap_base + (size_t)rs.frame_parity * rs.snap_stride : nullptr,
+                                      to_peer ? &rs.rctl.p->peer_parity : nullptr, to_peer ? (unsigned long long)rs.frame.n : 0ull};
+            rs.snapshot_taken = snap.dst != nullptr;
+#define GS_BLEND2D(FMT, SC) gs_launch(k_blend2d<FMT, SC>, grid, 128 * SC * SC, 0, st, rs.ranges.p, rs.list.p, rs.surfels.p, tiles_x, tiles_y, coarse_x, rank, world, (int)p.width, (int)p.height, p.flip_y, target, rs.tile_order.p, snap)
+            if (tshift == kTileShift) { if (p.frame_format == GS_FRAME_RGBA8) GS_BLEND2D(GS_FRAME_RGBA8, 1); else GS_BLEND2D(GS_FRAME_RGBA32F, 1); }
+            else { if (p.frame_format == GS_FRAME_RGBA8) GS_BLEND2D(GS_FRAME_RGBA8, 2); else GS_BLEND2D(GS_FRAME_RGBA32F, 2); }
+#undef GS_BLEND2D
+            ++launches;
+            prof.mark("k_blend2d", st);
+        } else if (rs.blend_version >= 2 || tshift != kTileShift) {
             const bool to_peer = peer_mode && rs.peer_attached;
             const StatusSnapshot snap{rs.snap_sort_ctl, reinterpret_cast<const uint32_t *>(rs.rctl.p),
                                       (rs.snap_base && rs.snap_sort_ctl) ? rs.snap_base + (size_t)rs.frame_parity * rs.snap_stride : nullptr,
@@ -1702,8 +1750,10 @@ static int raster_render(RasterState &rs, const gs_config &c, const gs_uniforms 
             gs_launch(k_blend<GS_FRAME_RGBA8>, grid, kBlendThreads, 0, st, rs.ranges.p, rs.list.p, rs.records.p, tiles_x, tiles_y, coarse_x, rank, world, (int)p.width, (int)p.height, p.flip_y, target, rs.tile_order.p);
         else
             gs_launch(k_blend<GS_FRAME_RGBA32F>, grid, kBlendThreads, 0, st, rs.ranges.p, rs.list.p, rs.records.p, tiles_x, tiles_y, coarse_x, rank, world, (int)p.width, (int)p.height, p.flip_y, target, rs.tile_order.p);
-        ++launches;
-        prof.mark("k_blend", st);
+        if (rs.render_mode != GS_RENDER_MODE_2D) {
+            ++launches;
+            prof.mark("k_blend", st);
+        }
         if (peer_mode && rs.peer_attached) { k_peer_signal<<<1, 1, 0, st>>>(rs.peer_sync); ++launches; }
         if (peer_mode && rs.peer_root) { k_peer_wait_arrived<<<1, 1, 0, st>>>(rs.peer_sync, rs.rctl.p, world - 1); ++launches; prof.mark("k_peer_wait_arrived", st); }
     }
@@ -1728,7 +1778,20 @@ static int raster_subset(RasterState &rs, const gs_config &c, const uint32_t *d_
     return GS_OK;
 }
 
+// 2D: re-run the projection with the last frame's parameters, exporting the vertex-stage outputs
+static int raster_read_projected_2d(RasterState &rs, gs_projected_surfel *out, uint32_t count, cudaStream_t st) {
+    if (rs.render_mode != GS_RENDER_MODE_2D) { snprintf(raster_err(), 512, "gs_read_projected_2d on a ThreeD engine (splat_render_mode 0)"); return GS_ERR_BAD_ARG; }
+    if (!rs.uploaded) { snprintf(raster_err(), 512, "gs_read_projected_2d before gs_upload_splat_data"); return GS_ERR_NOT_READY; }
+    if (count > rs.uploaded) { snprintf(raster_err(), 512, "count %u > uploaded %u", count, rs.uploaded); return GS_ERR_CAPACITY; }
+    RCU(rs.exported2d.ensure(rs.uploaded));
+    launch_project2d<true>(rs, rs.uploaded, st, rs.exported2d.p);
+    RCU(cudaGetLastError());
+    RCU(cudaMemcpyAsync(out, rs.exported2d.p, (size_t)count * sizeof(gs_projected_surfel), cudaMemcpyDeviceToHost, st));
+    return GS_OK;
+}
+
 static int raster_read_projected(RasterState &rs, gs_projected_splat *out, uint32_t count, cudaStream_t st) {
+    if (rs.render_mode == GS_RENDER_MODE_2D) { snprintf(raster_err(), 512, "gs_read_projected on a TwoD (surfel) engine: use gs_read_projected_2d"); return GS_ERR_BAD_ARG; }
     if (count > rs.uploaded) { snprintf(raster_err(), 512, "count %u > uploaded %u", count, rs.uploaded); return GS_ERR_CAPACITY; }
     RCU(rs.exported.ensure(count));
     if (count) k_export_projected<<<(count + 255) / 256, 256, 0, st>>>(rs.records.p, rs.rects.p, count, rs.exported.p);

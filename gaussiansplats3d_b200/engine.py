@@ -85,7 +85,8 @@ class Engine:
 
     def __init__(self, max_splat_count: int, *, device: int = 0, distance_map_range: int = 1 << 16,
                  integer_based_sort: bool = True, dynamic_mode: bool = False, max_width: int = 0, max_height: int = 0,
-                 rank: int = 0, world_size: int = 1):
+                 rank: int = 0, world_size: int = 1, splat_render_mode: int = N.GS_RENDER_MODE_3D):
+        """`splat_render_mode`: SplatRenderMode.ThreeD (0) or TwoD (1, 2D Gaussian surfels), fixed for the engine's lifetime."""
         self._lib = N.load()
         cfg = N.gs_config()
         cfg.struct_size = C.sizeof(N.gs_config)
@@ -96,6 +97,7 @@ class Engine:
         cfg.dynamic_mode = 1 if dynamic_mode else 0
         cfg.max_width, cfg.max_height = max_width, max_height
         cfg.rank, cfg.world_size = rank, world_size
+        cfg.splat_render_mode = int(splat_render_mode)
         self.cfg = cfg
         self._h = C.c_void_p()
         N.check(self._lib.gs_create(C.byref(cfg), C.byref(self._h)), "gs_create")
@@ -103,6 +105,7 @@ class Engine:
         self.integer_based_sort = integer_based_sort
         self.dynamic_mode = dynamic_mode
         self.rank, self.world_size = rank, world_size
+        self.splat_render_mode = int(splat_render_mode)
         self._keep: list = []
 
     # -- lifetime -------------------------------------------------------------------------------------------
@@ -236,21 +239,29 @@ class Engine:
         return out
 
     # -- rasteriser --------------------------------------------------------------------------------------------
-    def upload_splat_data(self, centers_colors: np.ndarray, covariances: np.ndarray, sh: np.ndarray | None = None,
-                          sh_degree: int = 0, scene_indexes: np.ndarray | None = None, start: int = 0) -> None:
+    def upload_splat_data(self, centers_colors: np.ndarray, covariances: np.ndarray | None, sh: np.ndarray | None = None,
+                          sh_degree: int = 0, scene_indexes: np.ndarray | None = None, start: int = 0, *,
+                          scale_rotations: np.ndarray | None = None) -> None:
+        """`scale_rotations` (f32 [n, 6] = sx sy sz qx qy qz): the data a TwoD engine renders from; it ignores `covariances`."""
         cc = np.ascontiguousarray(centers_colors, dtype=np.uint32).reshape(-1, 4)
         d = N.gs_splat_data()
         d.struct_size = C.sizeof(N.gs_splat_data)
         d.from_, d.count = start, cc.shape[0]
         d.centers_colors = N.ptr(cc)
-        cov = np.ascontiguousarray(covariances)
-        if cov.dtype == np.float16:
-            d.cov_format = N.GS_COV_F16
-        else:
-            cov = np.ascontiguousarray(cov, dtype=np.float32)
-            d.cov_format = N.GS_COV_F32
-        d.covariances = N.ptr(cov)
-        keep = [cc, cov]
+        keep = [cc]
+        if covariances is not None:
+            cov = np.ascontiguousarray(covariances)
+            if cov.dtype == np.float16:
+                d.cov_format = N.GS_COV_F16
+            else:
+                cov = np.ascontiguousarray(cov, dtype=np.float32)
+                d.cov_format = N.GS_COV_F32
+            d.covariances = N.ptr(cov)
+            keep.append(cov)
+        if scale_rotations is not None:
+            sr = np.ascontiguousarray(scale_rotations, dtype=np.float32).reshape(-1, 6)
+            d.scale_rotations = N.ptr(sr)
+            keep.append(sr)
         d.sh_degree = sh_degree if sh is not None else 0
         d.sh_format = N.GS_SH_NONE
         if sh is not None and sh_degree > 0:
@@ -393,6 +404,12 @@ class Engine:
     def read_projected(self, count: int) -> np.ndarray:
         out = np.empty(count, N.PROJECTED_DTYPE)
         N.check(self._lib.gs_read_projected(self._h, N.ptr(out), count), "gs_read_projected")
+        return out
+
+    def read_projected_2d(self, count: int) -> np.ndarray:
+        """TwoD engines: the vertex-stage output of every splat for the last frame's camera (gs_read_projected_2d)."""
+        out = np.empty(count, N.PROJECTED_SURFEL_DTYPE)
+        N.check(self._lib.gs_read_projected_2d(self._h, N.ptr(out), count), "gs_read_projected_2d")
         return out
 
     # -- device access -------------------------------------------------------------------------------------------

@@ -174,6 +174,73 @@ def transform_scene(raw: RawScene, transform16) -> tuple[RawScene, np.ndarray]:
     return RawScene(centers, raw.scales, raw.rotations, raw.colors, sh, raw.sh_degree), m[:3, :3].copy()
 
 
+def _quaternion_from_rotation(m11, m12, m13, m21, m22, m23, m31, m32, m33):
+    """Quaternion.setFromRotationMatrix (three r160), vectorised in float64; returns x, y, z, w."""
+    t = m11 + m22 + m33
+    x, y, z, w = (np.empty_like(t) for _ in range(4))
+    a = t > 0
+    b = ~a & (m11 > m22) & (m11 > m33)
+    c = ~a & ~b & (m22 > m33)
+    d = ~a & ~b & ~c
+    with np.errstate(divide="ignore", invalid="ignore"):
+        k = 0.5 / np.sqrt(t + 1.0)
+        w[a], x[a], y[a], z[a] = (0.25 / k)[a], ((m32 - m23) * k)[a], ((m13 - m31) * k)[a], ((m21 - m12) * k)[a]
+        k = 2.0 * np.sqrt(1.0 + m11 - m22 - m33)
+        w[b], x[b], y[b], z[b] = ((m32 - m23) / k)[b], (0.25 * k)[b], ((m12 + m21) / k)[b], ((m13 + m31) / k)[b]
+        k = 2.0 * np.sqrt(1.0 + m22 - m11 - m33)
+        w[c], x[c], y[c], z[c] = ((m13 - m31) / k)[c], ((m12 + m21) / k)[c], (0.25 * k)[c], ((m23 + m32) / k)[c]
+        k = 2.0 * np.sqrt(1.0 + m33 - m11 - m22)
+        w[d], x[d], y[d], z[d] = ((m21 - m12) / k)[d], ((m13 + m31) / k)[d], ((m23 + m32) / k)[d], (0.25 * k)[d]
+    return x, y, z, w
+
+
+def _normalize_quaternion(x, y, z, w):
+    """Quaternion.normalize: multiply by 1 / length; a zero quaternion becomes (0, 0, 0, 1)."""
+    ln = np.sqrt(x * x + y * y + z * z + w * w)
+    zero = ln == 0
+    with np.errstate(divide="ignore"):
+        il = 1.0 / ln
+    x, y, z, w = x * il, y * il, z * il, w * il
+    x[zero], y[zero], z[zero], w[zero] = 0.0, 0.0, 0.0, 1.0
+    return x, y, z, w
+
+
+def compute_scale_rotations(scales: np.ndarray, rotations_xyzw: np.ndarray, transform16=None, scale_z: float = 1.0) -> np.ndarray:
+    """The TwoD mode's scale/rotation texture: SplatBuffer.fillSplatScaleRotationArray (SplatBuffer.js:349-438) with the z scale
+    overridden to `scale_z` (SplatMesh.js:1856-1863), packed 6 x f32 per splat [sx sy sz qx qy qz] like
+    SplatMesh.updateScaleRotationsPaddedData (SplatMesh.js:1150-1170).  float64 in three.js's operation order: the quaternion is
+    normalised; with a scene transform the matrix transform * R * S is decomposed (Matrix4.decompose) and the quaternion normalised
+    again; finally w is made non-negative (ensurePositiveW)."""
+    n = scales.shape[0]
+    sx, sy = scales[:, 0].astype(np.float64), scales[:, 1].astype(np.float64)
+    sz = np.full(n, float(scale_z))
+    x, y, z, w = _normalize_quaternion(*(rotations_xyzw[:, k].astype(np.float64) for k in range(4)))
+    if transform16 is not None:
+        e = [float(v) for v in np.asarray(transform16, np.float64).reshape(16)]
+        x2, y2, z2 = x + x, y + y, z + z     # makeRotationFromQuaternion, then the columns times makeScale's diagonal (exact)
+        xx, xy, xz, yy, yz, zz, wx, wy, wz = x * x2, x * y2, x * z2, y * y2, y * z2, z * z2, w * x2, w * y2, w * z2
+        r = [[1 - (yy + zz), xy - wz, xz + wy], [xy + wz, 1 - (xx + zz), yz - wx], [xz - wy, yz + wx, 1 - (xx + yy)]]
+        rs = [[r[i][j] * (sx, sy, sz)[j] for j in range(3)] for i in range(3)]
+        t = [[e[0], e[4], e[8]], [e[1], e[5], e[9]], [e[2], e[6], e[10]]]
+        # Matrix4.multiplyMatrices(transform, R S): left-to-right sums (the fourth term, t[i][3] * 0, adds an exact zero)
+        m = [[(t[i][0] * rs[0][j] + t[i][1] * rs[1][j]) + t[i][2] * rs[2][j] for j in range(3)] for i in range(3)]
+        # Matrix4.decompose
+        dsx = np.sqrt(m[0][0] * m[0][0] + m[1][0] * m[1][0] + m[2][0] * m[2][0])
+        dsy = np.sqrt(m[0][1] * m[0][1] + m[1][1] * m[1][1] + m[2][1] * m[2][1])
+        dsz = np.sqrt(m[0][2] * m[0][2] + m[1][2] * m[1][2] + m[2][2] * m[2][2])
+        det = (-m[0][2] * m[1][1] * m[2][0] - m[0][0] * m[1][2] * m[2][1] + m[0][0] * m[1][1] * m[2][2]
+               + m[0][2] * m[1][0] * m[2][1] - m[0][1] * m[1][0] * m[2][2] + m[0][1] * m[1][2] * m[2][0])
+        dsx = np.where(det < 0, -dsx, dsx)
+        isx, isy, isz = 1.0 / dsx, 1.0 / dsy, 1.0 / dsz
+        x, y, z, w = _quaternion_from_rotation(m[0][0] * isx, m[0][1] * isy, m[0][2] * isz, m[1][0] * isx, m[1][1] * isy, m[1][2] * isz,
+                                               m[2][0] * isx, m[2][1] * isy, m[2][2] * isz)
+        x, y, z, w = _normalize_quaternion(x, y, z, w)
+        sx, sy, sz = dsx, dsy, dsz
+    flip = np.where(w < 0, -1.0, 1.0)
+    out = np.stack([sx, sy, sz, x * flip, y * flip, z * flip], 1)
+    return out.astype(np.float32)
+
+
 def pack_centers_colors(centers: np.ndarray, colors: np.ndarray, minimum_alpha: int = 1) -> np.ndarray:
     """SplatMesh.updateCenterColorsPaddedData (SplatMesh.js:1143-1153) + fillSplatColorArray's alpha floor
     (SplatBuffer.js:541-542): uvec4 {r | g<<8 | b<<16 | a<<24, bits(x), bits(y), bits(z)}."""
@@ -211,16 +278,23 @@ class PackedScene:
     sh_degree: int
     int_centers: np.ndarray      # i32 [n,4]
     count: int
+    scale_rotations: np.ndarray | None = None   # f32 [n,6], TwoD render mode only (instead of covariances)
 
 
 def pack_scene(raw: RawScene, *, half_covariances: bool = False, sh_format: str = "f16", minimum_alpha: int = 1,
-               sh8_range: tuple[float, float] = (-1.5, 1.5), transform16=None) -> PackedScene:
-    """`transform16` (column-major 4x4): the static scene transform baked into centres, covariances and SH (non-dynamic meshes)."""
+               sh8_range: tuple[float, float] = (-1.5, 1.5), transform16=None, render_mode: int = 0) -> PackedScene:
+    """`transform16` (column-major 4x4): the static scene transform baked into centres, covariances and SH (non-dynamic meshes).
+    `render_mode` 1 (SplatRenderMode.TwoD): the scale/rotation texture is built instead of the covariances (SplatMesh.js:1853-1870)."""
     t3 = None
+    srot = None
+    if render_mode == 1:
+        srot = compute_scale_rotations(raw.scales, raw.rotations, transform16)
     if transform16 is not None:
         raw, t3 = transform_scene(raw, transform16)
-    cov = compute_covariances(raw.scales, raw.rotations, t3)
-    if half_covariances:  # halfPrecisionCovariancesOnGPU
+    cov = None
+    if render_mode != 1:
+        cov = compute_covariances(raw.scales, raw.rotations, t3)
+    if half_covariances and cov is not None:  # halfPrecisionCovariancesOnGPU
         cov = cov.astype(np.float16)
     sh = None
     if raw.sh is not None and raw.sh_degree > 0:
@@ -233,7 +307,7 @@ def pack_scene(raw: RawScene, *, half_covariances: bool = False, sh_format: str 
         else:
             sh = flat.astype(np.float32)
     return PackedScene(pack_centers_colors(raw.centers, raw.colors, minimum_alpha), cov, sh, raw.sh_degree if sh is not None else 0,
-                       integer_centers(raw.centers), raw.count)
+                       integer_centers(raw.centers), raw.count, srot)
 
 
 # Cameras of the reference's demo pages (demo/bonsai.html:38-41, demo/garden.html:38-41) and the Viewer default

@@ -27,13 +27,20 @@ from .splat_tree import SplatTree, fov_cosines
 THREE_CAMERA_FOV = 50  # Viewer.js:30
 
 
+class SplatRenderMode:
+    """src/SplatRenderMode.js: the Viewer option `splatRenderMode` (Viewer.js:199-202)."""
+    ThreeD = 0
+    TwoD = 1
+
+
 class SplatMesh:
     """Owns the GPU-side splat data of one (static) scene and the uniforms of the splat material."""
 
     def __init__(self, *, dynamicMode=False, halfPrecisionCovariancesOnGPU=False, devicePixelRatio=1.0, antialiased=False,
                  maxScreenSpaceSplatSize=1024, splatScale=1.0, pointCloudModeEnabled=False, sphericalHarmonicsDegree=0,
-                 kernel2DSize=0.3, enableOptionalEffects=False):
+                 kernel2DSize=0.3, enableOptionalEffects=False, splatRenderMode=SplatRenderMode.ThreeD):
         self.dynamicMode = dynamicMode
+        self.splatRenderMode = int(splatRenderMode)
         self.halfPrecisionCovariancesOnGPU = halfPrecisionCovariancesOnGPU
         self.devicePixelRatio = devicePixelRatio
         self.antialiased = antialiased
@@ -76,7 +83,8 @@ class SplatMesh:
             ncoef = 0 if degree == 0 else (3 if degree == 1 else 8)
             raw_scene = RawScene(raw_scene.centers, raw_scene.scales, raw_scene.rotations, raw_scene.colors,
                                  None if degree == 0 else raw_scene.sh[:, :ncoef], degree)
-        self.packed = pack_scene(raw_scene, half_covariances=self.halfPrecisionCovariancesOnGPU, sh_format=sh_format, transform16=transform16)
+        self.packed = pack_scene(raw_scene, half_covariances=self.halfPrecisionCovariancesOnGPU, sh_format=sh_format, transform16=transform16,
+                                 render_mode=self.splatRenderMode)
 
     def fillTransformsArray(self) -> np.ndarray:  # noqa: N802  SplatMesh.js:1660-1673
         """f32[32 x 16] for the sorter ('transforms' of the sort message) and the vertex stage (`transforms` uniform)."""
@@ -107,7 +115,7 @@ class SplatMesh:
         """The WebGL renderer of the reference (SplatMesh.js:1300-1340) becomes the CUDA engine; uploads the 'textures'."""
         self.engine = engine
         p = self.packed
-        engine.upload_splat_data(p.centers_colors, p.covariances, p.sh, p.sh_degree)
+        engine.upload_splat_data(p.centers_colors, p.covariances, p.sh, p.sh_degree, scale_rotations=p.scale_rotations)
 
     def updateRenderIndexes(self, globalIndexes: np.ndarray | None, renderSplatCount: int) -> None:  # noqa: N802,N803
         """SplatMesh.js:1228-1235.  globalIndexes None = keep the order the engine's last sort left on the device."""
@@ -144,6 +152,9 @@ class Viewer:
         self.focalAdjustment = float(o.get("focalAdjustment", 1.0))
         self.maxScreenSpaceSplatSize = float(o.get("maxScreenSpaceSplatSize", 1024))
         self.halfPrecisionCovariancesOnGPU = bool(o.get("halfPrecisionCovariancesOnGPU", False))
+        self.splatRenderMode = int(o.get("splatRenderMode", SplatRenderMode.ThreeD))      # Viewer.js:199-202
+        if self.splatRenderMode not in (SplatRenderMode.ThreeD, SplatRenderMode.TwoD):
+            raise ValueError(f"splatRenderMode {self.splatRenderMode} is neither SplatRenderMode.ThreeD nor TwoD")
         prec = int(o.get("splatSortDistanceMapPrecision", DefaultSplatSortDistanceMapPrecision))
         self.splatSortDistanceMapPrecision = int(np.clip(prec, 10, 20 if self.integerBasedSort else 24))  # Viewer.js:207-210
         self.device = int(o.get("device", 0))
@@ -177,13 +188,14 @@ class Viewer:
         self.splatMesh = SplatMesh(dynamicMode=self.dynamicScene, halfPrecisionCovariancesOnGPU=self.halfPrecisionCovariancesOnGPU,
                                    devicePixelRatio=self.devicePixelRatio, antialiased=self.antialiased,
                                    maxScreenSpaceSplatSize=self.maxScreenSpaceSplatSize, sphericalHarmonicsDegree=self.sphericalHarmonicsDegree,
-                                   kernel2DSize=self.kernel2DSize)
+                                   kernel2DSize=self.kernel2DSize, splatRenderMode=self.splatRenderMode)
         identity = tuple(position) == (0.0, 0.0, 0.0) and tuple(rotation) == (0.0, 0.0, 0.0, 1.0) and tuple(scale) == (1.0, 1.0, 1.0)
         self.splatMesh.build(raw_scene, transform16=None if identity else TM.compose(position, rotation, scale))
         n = self.splatMesh.getSplatCount()
         self.engine = Engine(n, device=self.device, distance_map_range=1 << self.splatSortDistanceMapPrecision,
                              integer_based_sort=self.integerBasedSort, dynamic_mode=self.dynamicScene,
-                             max_width=self.renderWidth, max_height=self.renderHeight, rank=self.rank, world_size=self.world_size)
+                             max_width=self.renderWidth, max_height=self.renderHeight, rank=self.rank, world_size=self.world_size,
+                             splat_render_mode=self.splatRenderMode)
         self.splatMesh.setRenderer(self.engine)
         centers = (self.splatMesh.getIntegerCenters(0, n - 1, True) if self.integerBasedSort else self.splatMesh.getFloatCenters(0, n - 1, True))
         if separate_sort_worker:
@@ -209,10 +221,10 @@ class Viewer:
         self.splatMesh = SplatMesh(dynamicMode=False, halfPrecisionCovariancesOnGPU=self.halfPrecisionCovariancesOnGPU,
                                    devicePixelRatio=self.devicePixelRatio, antialiased=self.antialiased,
                                    maxScreenSpaceSplatSize=self.maxScreenSpaceSplatSize, sphericalHarmonicsDegree=self.sphericalHarmonicsDegree,
-                                   kernel2DSize=self.kernel2DSize)
+                                   kernel2DSize=self.kernel2DSize, splatRenderMode=self.splatRenderMode)
         self.engine = Engine(n, device=self.device, distance_map_range=1 << self.splatSortDistanceMapPrecision,
                              integer_based_sort=self.integerBasedSort, dynamic_mode=False, max_width=self.renderWidth, max_height=self.renderHeight,
-                             rank=self.rank, world_size=self.world_size)
+                             rank=self.rank, world_size=self.world_size, splat_render_mode=self.splatRenderMode)
         identity = tuple(position) == (0.0, 0.0, 0.0) and tuple(rotation) == (0.0, 0.0, 0.0, 1.0) and tuple(scale) == (1.0, 1.0, 1.0)
         info = self.engine.upload_ksplat(data, half_covariances=self.halfPrecisionCovariancesOnGPU,
                                          transform16=None if identity else TM.compose(position, rotation, scale))

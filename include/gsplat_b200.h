@@ -77,6 +77,11 @@ GS_API void sortIndexes(unsigned int *indexes, void *centers, void *precomputedD
  * ---------------------------------------------------------------------------------------------------------- */
 typedef struct gs_engine gs_engine;
 
+typedef enum gs_render_mode {
+    GS_RENDER_MODE_3D = 0,   /* SplatRenderMode.ThreeD: SplatMaterial3D (covariances)                                    */
+    GS_RENDER_MODE_2D = 1    /* SplatRenderMode.TwoD: 2D Gaussian surfels, SplatMaterial2D (scale + rotation)            */
+} gs_render_mode;
+
 typedef struct gs_config {
     uint32_t struct_size;           /* sizeof(gs_config), for ABI growth                                        */
     int32_t device;                 /* CUDA device ordinal                                                       */
@@ -84,7 +89,9 @@ typedef struct gs_config {
     uint32_t distance_map_range;    /* 1 << splatSortDistanceMapPrecision        SortWorker.js:243, Constants.js:3 */
     uint8_t integer_based_sort;     /* Viewer option integerBasedSort            Viewer.js:95-98                 */
     uint8_t dynamic_mode;           /* Viewer option dynamicScene                SortWorker.js:120               */
-    uint8_t reserved0[2];
+    uint8_t splat_render_mode;      /* Viewer option splatRenderMode (SplatRenderMode.js, Viewer.js:199-202), fixed
+                                       for the engine's lifetime like the reference's material: GS_RENDER_MODE_*     */
+    uint8_t reserved0;
     uint32_t max_width, max_height; /* largest framebuffer gs_render will be asked for (0,0: sort only)          */
     /* multi-GPU sharding (one engine per process per GPU): this engine rasterises the 128x64-pixel coarse tiles
      * (cx, cy) with (cx + cy) % world_size == rank and leaves every other pixel of its frame zero, so the ranks'
@@ -161,13 +168,20 @@ typedef struct gs_splat_data {
     int32_t sh_format;                /* gs_sh_format                                                             */
     uint32_t sh_degree;               /* 0, 1 (9 values) or 2 (24 values)                                         */
     const uint32_t *scene_indexes;    /* u32 per splat or NULL (single scene)                                     */
+    /* appended (callers built against the older, shorter struct are recognised by struct_size):                          */
+    const float *scale_rotations;     /* GS_RENDER_MODE_2D engines: 6 x f32 per splat [sx sy sz qx qy qz], qw rebuilt as
+                                         sqrt(1 - x^2 - y^2 - z^2) (SplatMesh.updateScaleRotationsPaddedData :1150-1170).
+                                         Required there, and `covariances` is then ignored; unused by 3D engines.           */
 } gs_splat_data;
 
 GS_API int gs_upload_splat_data(gs_engine *e, const gs_splat_data *d);
 
 /* `.ksplat` buffer (the SplatBuffer container, src/loaders/SplatBuffer.js:819-941, KSplatLoader.loadFromFileData) decoded ON THE
  * GPU into everything above at once: centres+colours, covariances, spherical harmonics AND the sorter's centres
- * (= new SplatBuffer(fileData) + SplatMesh.build + the 'centers' message).  Compression levels 0/1/2, SH degree 0/1/2.        */
+ * (= new SplatBuffer(fileData) + SplatMesh.build + the 'centers' message).  Compression levels 0/1/2, SH degree 0/1/2.
+ * A GS_RENDER_MODE_2D engine decodes the scale/rotation texture (fillSplatScaleRotationArray, SplatBuffer.js:349-438, z scale
+ * overridden to 1 as SplatMesh.js:1856-1863 does, read at the file's level: 2^-24 for levels 1 and 2) instead of covariances;
+ * `half_covariances` has no meaning there.                                                                                       */
 typedef struct gs_ksplat_options {
     uint32_t struct_size;
     uint32_t minimum_alpha;          /* splatAlphaRemovalThreshold (Viewer.js), default 1: alpha below it renders as 0            */
@@ -263,9 +277,10 @@ typedef enum gs_buffer_id {
     GS_BUF_FRAME = 1,          /* last rendered frame in the requested format                                     */
     GS_BUF_CENTERS = 2,
     GS_BUF_DISTANCES = 3,      /* i32[render_count] scratch (= mappedDistances)                                   */
-    GS_BUF_SPLAT_RECORDS = 4,  /* per-splat projected records (engine-internal 48-byte layout)                    */
+    GS_BUF_SPLAT_RECORDS = 4,  /* per-splat projected records (engine-internal layout: 48 B, 2D engines 96 B)     */
     GS_BUF_INDEXES_TO_SORT = 5,/* u32[max_splat_count] staging for indexesToSort                                  */
-    GS_BUF_CENTERS_COLORS = 6, GS_BUF_COVARIANCES = 7, GS_BUF_SH = 8   /* the uploaded / decoded splat data (gs_read_buffer only) */
+    GS_BUF_CENTERS_COLORS = 6, GS_BUF_COVARIANCES = 7, GS_BUF_SH = 8,  /* the uploaded / decoded splat data (gs_read_buffer only) */
+    GS_BUF_SCALE_ROTATIONS = 9 /* 2D engines: 6 x f32 per splat, as gs_splat_data.scale_rotations (gs_read_buffer only)          */
 } gs_buffer_id;
 GS_API int gs_buffer_dev(gs_engine *e, int buffer_id, void **ptr_dev, size_t *bytes);
 GS_API int gs_read_buffer(gs_engine *e, int buffer_id, void *out, size_t offset, size_t bytes); /* D2H copy, for tests / tools */
@@ -319,6 +334,23 @@ typedef struct gs_projected_splat {
     uint32_t valid;      /* 0 = culled / dropped                                                                  */
 } gs_projected_splat;
 GS_API int gs_read_projected(gs_engine *e, gs_projected_splat *out, uint32_t count); /* splat order */
+
+/* Per-splat output of the 2D (surfel) vertex stage, SplatMaterial2D.js:96-235, for parity tests of GS_RENDER_MODE_2D engines.
+ * Re-runs the projection with the parameters of the engine's last frame: the per-splat records and tile rects are rewritten with
+ * the same values, and the statistics gs_last_timings reports are left as they are.  gs_read_projected returns GS_ERR_BAD_ARG on a
+ * TwoD engine (it has no 3D records), as gs_read_projected_2d does on a ThreeD engine.                                           */
+typedef struct gs_projected_surfel {
+    float T[9];          /* vT = T = transpose(splat2World) * world2ndc * ndc2pix, column-major: Tu = T[0..2], Tv, Tw     */
+    float qcx, qcy;      /* vQuadCenter: NDC units in the eigen branch (as the reference), pixels in the fallback          */
+    float cx, cy;        /* quad centre, pixels, GL window coordinates                                                     */
+    float h1x, h1y;      /* quad half-edges, pixels: corners = c +- h1 +- h2                                               */
+    float h2x, h2y;
+    float r, g, b, a;    /* vColor                                                                                         */
+    float ndc_z;
+    uint32_t branch;     /* 0 = eigen-aligned quad (:199-234), 1 = screen-aligned fallback square (:159-189)               */
+    uint32_t valid;      /* 0 = culled / dropped (incl. |distance| < 1e-5, where the reference leaves gl_Position unset)   */
+} gs_projected_surfel;
+GS_API int gs_read_projected_2d(gs_engine *e, gs_projected_surfel *out, uint32_t count); /* splat order */
 
 typedef struct gs_timings {
     float depth_ms, bucket_ms, scatter_ms, sort_total_ms;

@@ -59,7 +59,8 @@ class B200SortWorker {
             this.dynamicMode = i.dynamicMode;
             this.engine = addon.create({ maxSplatCount: i.splatCount, distanceMapRange: i.distanceMapRange,
                                          integerBasedSort: i.integerBasedSort ? 1 : 0, dynamicMode: i.dynamicMode ? 1 : 0,
-                                         maxWidth: i.maxWidth || 0, maxHeight: i.maxHeight || 0, device: i.device || 0 });
+                                         maxWidth: i.maxWidth || 0, maxHeight: i.maxHeight || 0, device: i.device || 0,
+                                         splatRenderMode: i.splatRenderMode || 0 });   // Viewer option splatRenderMode (Viewer.js:199-202)
             const msg = { sortSetupPhase1Complete: true };
             if (this.useSharedMemory) {
                 const n = i.splatCount;

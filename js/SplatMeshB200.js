@@ -33,9 +33,19 @@ export class B200SplatRenderer {
         const shDegree = splatMesh.minSphericalHarmonicsDegree || 0;
         let shFormat = GS_SH_NONE;
         if (sh && shDegree > 0) shFormat = (sh instanceof Uint8Array) ? GS_SH_U8 : ((sh instanceof Uint16Array) ? GS_SH_F16 : GS_SH_F32);
+        // SplatRenderMode.TwoD (the engine was created with splatRenderMode: 1): the scale/rotation texture of
+        // SplatMesh.updateScaleRotationsPaddedData (SplatMesh.js:1150-1170), 6 floats per splat, instead of covariances
+        let scaleRotations = null;
+        if (splatMesh.splatRenderMode === 1) {
+            scaleRotations = new Float32Array(6 * n);
+            for (let i = 0; i < n; i++) {
+                for (let k = 0; k < 3; k++) scaleRotations[6 * i + k] = base.scales[3 * i + k];
+                for (let k = 0; k < 3; k++) scaleRotations[6 * i + 3 + k] = base.rotations[4 * i + k];
+            }
+        }
         addon.uploadSplatData(this.engine, {
-            from: 0, count: n, centersColors: cc,
-            covariances: base.covariances, covFormat: (base.covariances instanceof Uint16Array) ? 1 : GS_COV_F32,
+            from: 0, count: n, centersColors: cc, scaleRotations,
+            covariances: base.covariances || null, covFormat: (base.covariances instanceof Uint16Array) ? 1 : GS_COV_F32,
             sphericalHarmonics: shFormat === GS_SH_NONE ? null : sh, shFormat, shDegree,
             sceneIndexes: splatMesh.dynamicMode ? base.sceneIndexes : null,
         });

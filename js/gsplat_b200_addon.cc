@@ -197,6 +197,7 @@ FN(Create) {
     c.distance_map_range = to_u32(env, prop(env, a[0], "distanceMapRange"));
     c.integer_based_sort = (uint8_t)to_u32(env, prop(env, a[0], "integerBasedSort"), 1);
     c.dynamic_mode = (uint8_t)to_u32(env, prop(env, a[0], "dynamicMode"));
+    c.splat_render_mode = (uint8_t)to_u32(env, prop(env, a[0], "splatRenderMode"));   // SplatRenderMode.ThreeD = 0 / TwoD = 1
     c.max_width = to_u32(env, prop(env, a[0], "maxWidth"));
     c.max_height = to_u32(env, prop(env, a[0], "maxHeight"));
     c.rank = to_u32(env, prop(env, a[0], "rank"));
@@ -242,7 +243,7 @@ FN(ComputeDistances) { // (engine, modelViewProj[16] f64, sceneTransforms f64[51
     CHECK(gs_compute_distances(engine_of(env, a[0]), mvp, tr.empty() ? nullptr : tr.data(), to_u32(env, a[3]), typed_ptr(env, a[4])));
     return undefined(env);
 }
-FN(UploadSplatData) { // (engine, {from, count, centersColors, covariances, covFormat, sphericalHarmonics, shFormat, shDegree, sceneIndexes})
+FN(UploadSplatData) { // (engine, {from, count, centersColors, covariances, covFormat, sphericalHarmonics, shFormat, shDegree, sceneIndexes, scaleRotations})
     ARGS(2)
     gs_splat_data d; memset(&d, 0, sizeof(d)); d.struct_size = sizeof(d);
     d.from = to_u32(env, prop(env, a[1], "from"));
@@ -254,6 +255,7 @@ FN(UploadSplatData) { // (engine, {from, count, centersColors, covariances, covF
     d.sh_format = to_i32(env, prop(env, a[1], "shFormat"));
     d.sh_degree = to_u32(env, prop(env, a[1], "shDegree"));
     d.scene_indexes = (const uint32_t *)typed_ptr(env, prop(env, a[1], "sceneIndexes"));
+    d.scale_rotations = (const float *)typed_ptr(env, prop(env, a[1], "scaleRotations"));   // TwoD: the scale/rotation texture
     CHECK(gs_upload_splat_data(engine_of(env, a[0]), &d));
     return undefined(env);
 }
@@ -382,6 +384,14 @@ FN(ReadProjected) {   // (engine, count) -> ArrayBuffer of gs_projected_splat re
     CHECK(gs_read_projected(engine_of(env, a[0]), (gs_projected_splat *)data, n));
     return ab;
 }
+FN(ReadProjected2D) { // (engine, count) -> ArrayBuffer of gs_projected_surfel records (TwoD engines)
+    ARGS(2)
+    const uint32_t n = to_u32(env, a[1]);
+    void *data = nullptr; napi_value ab;
+    napi_create_arraybuffer(env, (size_t)n * sizeof(gs_projected_surfel), &data, &ab);
+    CHECK(gs_read_projected_2d(engine_of(env, a[0]), (gs_projected_surfel *)data, n));
+    return ab;
+}
 FN(LastTimings) {
     ARGS(1)
     gs_timings t; memset(&t, 0, sizeof(t));
@@ -426,7 +436,7 @@ static napi_value Init(napi_env env, napi_value exports) {
         EXPORT("readBuffer", ReadBuffer), EXPORT("stream", Stream), EXPORT("synchronize", Synchronize), EXPORT("peerExport", PeerExport),
         EXPORT("peerAttach", PeerAttach), EXPORT("shardExport", ShardExport), EXPORT("shardAttach", ShardAttach), EXPORT("shardAttachLocal", ShardAttachLocal),
         EXPORT("sortSharded", SortSharded), EXPORT("sortShardedAsync", SortShardedAsync), EXPORT("sortShardedFinish", SortShardedFinish),
-        EXPORT("hostAlloc", HostAlloc), EXPORT("hostFree", HostFree), EXPORT("readProjected", ReadProjected), EXPORT("lastTimings", LastTimings),
+        EXPORT("hostAlloc", HostAlloc), EXPORT("hostFree", HostFree), EXPORT("readProjected", ReadProjected), EXPORT("readProjected2D", ReadProjected2D), EXPORT("lastTimings", LastTimings),
         EXPORT("flushL2", FlushL2), EXPORT("setProfiling", SetProfiling), EXPORT("setGraphEnabled", SetGraphEnabled), EXPORT("kernelTimings", KernelTimings),
         EXPORT("eventCreate", EventCreate), EXPORT("eventRecord", EventRecord), EXPORT("eventElapsedMs", EventElapsedMs), EXPORT("eventDestroy", EventDestroy),
     };
