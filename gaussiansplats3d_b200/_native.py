@@ -27,7 +27,8 @@ GS_OK, GS_ERR_BAD_ARG, GS_ERR_NO_DEVICE, GS_ERR_CUDA, GS_ERR_DEGENERATE, GS_ERR_
 GS_COV_F32, GS_COV_F16 = 0, 1
 GS_SH_NONE, GS_SH_F16, GS_SH_U8, GS_SH_F32 = 0, 1, 2, 3
 GS_FRAME_RGBA32F, GS_FRAME_RGBA8 = 0, 1
-GS_BUF_SORTED_INDEXES, GS_BUF_FRAME, GS_BUF_CENTERS, GS_BUF_DISTANCES, GS_BUF_SPLAT_RECORDS, GS_BUF_INDEXES_TO_SORT, GS_BUF_CENTERS_COLORS, GS_BUF_COVARIANCES, GS_BUF_SH, GS_BUF_SCALE_ROTATIONS = range(10)
+GS_BUF_SORTED_INDEXES, GS_BUF_FRAME, GS_BUF_CENTERS, GS_BUF_DISTANCES, GS_BUF_SPLAT_RECORDS, GS_BUF_INDEXES_TO_SORT, GS_BUF_CENTERS_COLORS, GS_BUF_COVARIANCES, GS_BUF_SH, GS_BUF_SCALE_ROTATIONS, \
+    GS_BUF_TILE_RECTS, GS_BUF_TILE_RANGES, GS_BUF_TILE_LIST, GS_BUF_TILE_ORDER, GS_BUF_TILE_INFO = range(15)
 GS_RENDER_MODE_3D, GS_RENDER_MODE_2D = 0, 1
 
 

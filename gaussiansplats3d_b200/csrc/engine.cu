@@ -1395,7 +1395,17 @@ extern "C" int gs_read_buffer(gs_engine *e, int id, void *out, size_t offset, si
     if (rc) return rc;
     if (!out) return fail(GS_ERR_BAD_ARG, "gs_read_buffer: null");
     const unsigned char *p = nullptr; size_t cap = 0;
+    if (id == GS_BUF_TILE_INFO) {     // host-side values
+        const uint64_t info[4] = {e->rs.instance_capacity, e->rs.last_ncoarse, e->rs.last_tile_px, e->rs.last_bin_path};
+        if (offset + bytes > sizeof(info)) return fail(GS_ERR_CAPACITY, "gs_read_buffer: [%zu,%zu) outside the %zu-byte buffer", offset, offset + bytes, sizeof(info));
+        memcpy(out, (const unsigned char *)info + offset, bytes);
+        return GS_OK;
+    }
     switch (id) {
+        case GS_BUF_TILE_RECTS: p = (const unsigned char *)e->rs.rects.p; cap = e->rs.rects.n * sizeof(ushort4); break;
+        case GS_BUF_TILE_RANGES: p = (const unsigned char *)e->rs.ranges.p; cap = e->rs.ranges.n * sizeof(uint2); break;
+        case GS_BUF_TILE_LIST: p = (const unsigned char *)e->rs.list.p; cap = std::min<size_t>(e->rs.list.n, e->rs.instance_capacity) * 8; break;
+        case GS_BUF_TILE_ORDER: p = (const unsigned char *)e->rs.tile_order.p; cap = e->rs.tile_order.n * 4; break;
         case GS_BUF_CENTERS_COLORS: p = (const unsigned char *)e->rs.cc.p; cap = e->rs.cc.n * 16; break;
         case GS_BUF_COVARIANCES: p = e->rs.cov.p; cap = e->rs.cov.n; break;
         case GS_BUF_SH: p = e->rs.sh.p; cap = e->rs.sh.n; break;

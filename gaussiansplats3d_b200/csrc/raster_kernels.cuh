@@ -402,8 +402,10 @@ k_project(const uint4 *__restrict__ cc, const void *__restrict__ cov, const void
 constexpr int kCoarseW = 8, kCoarseH = 4, kCoarseShiftX = 3, kCoarseShiftY = 2;
 constexpr int kFinePerCoarse = kCoarseW * kCoarseH;   // 32 = bits of the mask
 
-// Ownership as a bitmask over the diagonal index cx + cy (< 128 for frames up to 8K): bit set = this rank's tile.  Avoids integer
-// division by a run-time world size in the per-splat binning kernels.
+// Ownership as a bitmask over the diagonal index cx + cy: bit set = this rank's tile.  Avoids integer division by a run-time world
+// size in the per-splat binning kernels.  The mask covers diagonals 0..127 only (7680x4320 reaches 62), so raster_render refuses a
+// sharded frame whose largest diagonal is 128 or more (kMaxOwnDiag) with GS_ERR_BAD_ARG instead of binning it wrongly.
+constexpr int kMaxOwnDiag = 127;
 struct OwnMask { unsigned long long lo, hi; };
 __host__ __device__ __forceinline__ bool own_diag(const OwnMask &m, int diag) {
     return ((diag < 64 ? m.lo >> diag : m.hi >> (diag - 64)) & 1ull) != 0ull;
@@ -709,9 +711,13 @@ k_bin_count(const uint32_t *__restrict__ order, uint32_t render_count_host, cons
 }
 
 // One CTA per coarse tile: where its list starts (all smaller tiles' totals) and the running offset of every chunk inside it.
+// On an overflowing frame k_bin_place stores only the slots below `capacity`; slot s holds the same instance either way, so the
+// tile ranges are clamped to the capacity and every blend reads written entries only.  total_instances stays UNclamped: it is the
+// count the host reports with GS_ERR_CAPACITY.
 __global__ void __launch_bounds__(1024)
 k_bin_scan(uint32_t *__restrict__ hist, uint32_t stride, uint32_t ranks_per_chunk, uint32_t render_count_host, const unsigned long long *__restrict__ n_dev,
-           const uint32_t *__restrict__ totals, uint32_t nt, uint2 *__restrict__ ranges, RasterControl *rctl, uint32_t *__restrict__ tile_order) {
+           const uint32_t *__restrict__ totals, uint32_t nt, uint2 *__restrict__ ranges, RasterControl *rctl, uint32_t *__restrict__ tile_order,
+           unsigned long long capacity) {
     pdl_enter();
     __shared__ uint32_t s_scan[40];
     __shared__ uint32_t s_carry;
@@ -733,7 +739,8 @@ k_bin_scan(uint32_t *__restrict__ hist, uint32_t stride, uint32_t ranks_per_chun
         if (threadIdx.x == 0) {
             s_carry = total;
             const uint32_t mine = totals[d];
-            ranges[d] = make_uint2(total, total + mine);
+            const uint32_t cap = (uint32_t)min(capacity, 0xffffffffull);
+            ranges[d] = make_uint2(min(total, cap), min(total + mine, cap));
             if (d == nt - 1) rctl->total_instances = (unsigned long long)total + mine;
         }
     }
@@ -1217,7 +1224,9 @@ k_blend2(const uint2 *__restrict__ ranges, const unsigned long long *__restrict_
         mbar_expect_tx(&s_mbar[b & 1u], bytes);
         bulk_g2s(&s_chunk[b & 1u][0], list + a0, bytes, &s_mbar[b & 1u]);
     };
-    const uint32_t nbatch = (rg.y - rg.x + BATCH - 1) / BATCH;
+    // the radix binning path marks an empty tile (0xffffffff, 0): no batch (the u32 difference would wrap to one batch, and a bulk copy
+    // would then be issued far outside the list)
+    const uint32_t nbatch = rg.y > rg.x ? (rg.y - rg.x + BATCH - 1) / BATCH : 0u;
     if (TMA && threadIdx.x == 0) { mbar_init(&s_mbar[0], 1); mbar_init(&s_mbar[1], 1); mbar_fence_init(); }
     __syncthreads();
     if (TMA && threadIdx.x == 0 && nbatch) issue(0);
@@ -1452,6 +1461,8 @@ struct RasterState {
     void *peer_frame = nullptr;          // others: rank 0's frame buffer mapped through CUDA IPC
     bool peer_root = false, peer_attached = false;
     unsigned long long instance_capacity = 0;
+    // binning of the last frame (GS_BUF_TILE_INFO): coarse tiles, fine-tile edge in px, path (2 = counting sort, 1 = radix sort)
+    uint32_t last_ncoarse = 0, last_tile_px = 0, last_bin_path = 0;
     uint32_t hist_stride = 0;
     int sm_count = 148;
     int last_format = GS_FRAME_RGBA32F;
@@ -1491,7 +1502,8 @@ static int raster_init(RasterState &rs, const gs_config &c, int sm_count) {
         rs.instance_capacity = (unsigned long long)(factor * (double)n) + 4ull * tiles + 65536ull;
         if (rs.instance_capacity > 0xfffffff0ull) rs.instance_capacity = 0xfffffff0ull;
         for (int i = 0; i < 2; ++i) { RCU(rs.ikeys[i].ensure(rs.instance_capacity)); RCU(rs.ivals[i].ensure(rs.instance_capacity)); }
-        RCU(rs.list.ensure(rs.instance_capacity));
+        // +2: k_blend2's bulk list copies start and end on an even entry, so a list ending at the capacity may read one entry beyond it
+        RCU(rs.list.ensure(rs.instance_capacity + 2));
         RCU(rs.ranges.ensure(65536));
         RCU(rs.tile_order.ensure(65536));
         RCU(rs.frame.ensure((size_t)c.max_width * (c.max_height + kTile) * 16));
@@ -1645,6 +1657,11 @@ static int raster_render(RasterState &rs, const gs_config &c, const gs_uniforms 
     const int coarse_x = (tiles_x + kCoarseW - 1) / kCoarseW, coarse_y = (tiles_y + kCoarseH - 1) / kCoarseH;
     const uint32_t ncoarse = (uint32_t)coarse_x * (uint32_t)coarse_y;
     if (ncoarse > 65536u) { snprintf(raster_err(), 512, "frame %ux%u needs %u coarse tiles (> 65536)", p.width, p.height, ncoarse); return GS_ERR_BAD_ARG; }
+    if (world > 1 && coarse_x - 1 + coarse_y - 1 > kMaxOwnDiag) {
+        snprintf(raster_err(), 512, "frame %ux%u is too long for sharded rendering: its coarse-tile diagonal cx + cy reaches %d (at most %d with world_size > 1)",
+                 p.width, p.height, coarse_x - 1 + coarse_y - 1, kMaxOwnDiag);
+        return GS_ERR_BAD_ARG;
+    }
     int tile_bits = 1;
     while ((1u << tile_bits) < std::max(ncoarse, 2u)) ++tile_bits;
     const PassPlan pl = make_plan_bits(tile_bits);
@@ -1670,6 +1687,7 @@ static int raster_render(RasterState &rs, const gs_config &c, const gs_uniforms 
     if (!(phases & 2)) { tm.kernel_launches = launches; return GS_OK; }
     rs.snapshot_taken = false;
     const bool bin2 = rs.bin_version >= 2 && ncoarse <= 256u;
+    rs.last_ncoarse = ncoarse; rs.last_tile_px = (uint32_t)tpx; rs.last_bin_path = bin2 ? 2u : 1u;
     if (p.render_count && local_tiles && bin2) {
         const OwnMask own = make_own_mask(rank, world);
         const int sharded = world > 1 ? 1 : 0;
@@ -1679,7 +1697,8 @@ static int raster_render(RasterState &rs, const gs_config &c, const gs_uniforms 
         if (rs.bin_cfg == 0) GS_BIN_COUNT(0); else GS_BIN_COUNT(1);
         ++launches;
         prof.mark("k_bin_count", st);
-        gs_launch(k_bin_scan, ncoarse, 1024, 0, st, rs.bin_hist.p, rs.bin_stride, (uint32_t)kBinRanks, p.render_count, order_count_dev, rs.bin_totals.p, ncoarse, rs.ranges.p, rs.rctl.p, rs.tile_order.p);
+        gs_launch(k_bin_scan, ncoarse, 1024, 0, st, rs.bin_hist.p, rs.bin_stride, (uint32_t)kBinRanks, p.render_count, order_count_dev, rs.bin_totals.p, ncoarse, rs.ranges.p, rs.rctl.p, rs.tile_order.p,
+                  rs.instance_capacity);
         ++launches;
         prof.mark("k_bin_scan", st);
         if (rs.bin_cfg == 0) GS_BIN_PLACE(0); else GS_BIN_PLACE(1);

@@ -336,7 +336,7 @@ k_blend2d(const uint2 *__restrict__ ranges, const unsigned long long *__restrict
     bool wdone = !__any_sync(0xffffffffu, fmaxf(lo2(T), hi2(T)) >= kTransmittanceCutoff);
     const uint2 rg = ranges[coarse];
     const uint32_t lt = lanemask_lt();
-    const uint32_t nbatch = (rg.y - rg.x + BATCH - 1) / BATCH;
+    const uint32_t nbatch = rg.y > rg.x ? (rg.y - rg.x + BATCH - 1) / BATCH : 0u;     // (0xffffffff, 0): an empty tile of the radix path
     for (uint32_t b = 0; b < nbatch; ++b) {
         const uint32_t base = rg.x + b * (uint32_t)BATCH;
         if (__syncthreads_and(wdone)) break;

@@ -280,7 +280,14 @@ typedef enum gs_buffer_id {
     GS_BUF_SPLAT_RECORDS = 4,  /* per-splat projected records (engine-internal layout: 48 B, 2D engines 96 B)     */
     GS_BUF_INDEXES_TO_SORT = 5,/* u32[max_splat_count] staging for indexesToSort                                  */
     GS_BUF_CENTERS_COLORS = 6, GS_BUF_COVARIANCES = 7, GS_BUF_SH = 8,  /* the uploaded / decoded splat data (gs_read_buffer only) */
-    GS_BUF_SCALE_ROTATIONS = 9 /* 2D engines: 6 x f32 per splat, as gs_splat_data.scale_rotations (gs_read_buffer only)          */
+    GS_BUF_SCALE_ROTATIONS = 9,/* 2D engines: 6 x f32 per splat, as gs_splat_data.scale_rotations (gs_read_buffer only)          */
+    /* Tile binning of the last rendered frame, for tests (gs_read_buffer only).  Coarse tiles are 8 x 4 fine tiles, numbered
+     * cy * coarse_x + cx; a list entry is (fine-tile mask << 32) | splat id, bit 8 * fy + fx = fine tile (fx, fy) of the coarse tile.    */
+    GS_BUF_TILE_RECTS = 10,    /* u16x4 per uploaded splat: inclusive fine-tile rect {x0, y0, x1, y1}; empty (x1 < x0) = not drawn    */
+    GS_BUF_TILE_RANGES = 11,   /* u32x2 per coarse tile: [first, end) of its list; clamped to the instance capacity               */
+    GS_BUF_TILE_LIST = 12,     /* u64 list entries, per coarse tile in draw order (up to the instance capacity)                   */
+    GS_BUF_TILE_ORDER = 13,    /* u32 per coarse tile: the blend's schedule of coarse tiles                                       */
+    GS_BUF_TILE_INFO = 14      /* u64[4]: instance capacity, coarse tiles, fine-tile edge in px, binning path (2 counting, 1 radix) */
 } gs_buffer_id;
 GS_API int gs_buffer_dev(gs_engine *e, int buffer_id, void **ptr_dev, size_t *bytes);
 GS_API int gs_read_buffer(gs_engine *e, int buffer_id, void *out, size_t offset, size_t bytes); /* D2H copy, for tests / tools */
